@@ -2,7 +2,7 @@
 """Benchmark of the D-MPNN hot path (BASELINE.json): molecules/sec, forward+backward, of the message-passing encoder +
 aggregation on synthetic molecule batches.
 
-    python bench.py [--config C2|C3|C4|C5] [--gpus N] [--steps K] [--warmup W] [--impl reference]
+    python bench.py [--config C2|C3|C4|C5] [--gpus N] [--steps K] [--warmup W] [--impl reference] [--dump-outputs DIR]
 
 Configurations (BASELINE.json `configs`; C1 is the reference's CPU plumbing case and lives in the tests):
   C2  10 k ~25-atom molecules / GPU, BondMessagePassing h=300 depth=3, bf16 tier, fused depth step   (default, weak scaling)
@@ -22,6 +22,11 @@ Prints ONE JSON line (rank 0):
  e2e_host_batch  (C2, N = 1) the same step fed with a complete host batch per step (bf16 features + int32 indices, 57 MB H2D)
  roofline      the dominant kernel: algorithmic bytes or flops / its CUDA-event duration vs the measured peak
  cpu_baseline  the oracle port (the reference's own op sequence on torch CPU) on the host cores, bounded sample
+
+`--dump-outputs DIR` writes the results of the last timed step of the path `value` measures: the per-atom hidden states
+`H` and the per-molecule aggregates `agg` (a fixed, seeded sample of rows when larger than 16 MB), the `loss` and every
+weight gradient `grad.<name>`, as float32 .npy files.  Inputs and weights are seeded, so two builds run with the same
+arguments can be compared array for array.
 
 `--impl reference` times that CPU implementation on the SAME workload (full batch per step) on the host's cores.
 """
@@ -354,12 +359,26 @@ def main_gpu(args):
     V_atoms, E_rows = resident.V.shape[0], resident.E.shape[0]
     n_tiles = resident._meta_host[_lib.META_N_TILES] if resident._meta_host else None
 
+    last = {}                                    # --dump-outputs: the latest step's results (static outputs under a graph)
+
     def fwd_bwd(bmg):
         bmg._layout = None                       # the device layout build is part of every step
         H = mp(bmg)
-        loss = agg(H, bmg.batch).float().square().mean()
+        a = agg(H, bmg.batch)
+        loss = a.float().square().mean()
         loss.backward()
+        if args.dump_outputs:
+            last.update(H=H.detach(), agg=a.detach(), loss=loss.detach())   # no autograd graph kept alive
         return loss
+
+    def snapshot():
+        """Host copies of what the timed path computed in its last step (taken after the timed region)."""
+        torch.cuda.synchronize()
+        out = {"H": sample_rows(last["H"]), "agg": sample_rows(last["agg"]),
+               "loss": last["loss"].detach().float().reshape(1).cpu().numpy()}
+        for k, p in mp.named_parameters():
+            out["grad." + k] = p.grad.detach().float().cpu().numpy()
+        return out
 
     def step_resident():
         zero_grads()
@@ -404,6 +423,7 @@ def main_gpu(args):
         ms = timed(step_resident, args.steps)
     launches = lib.dmpnn_launch_count() - l0
     step_events, engine.STEP_EVENTS = engine.STEP_EVENTS, None
+    dump = snapshot() if args.dump_outputs else None
     ms_per_step = ms / args.steps
     value = mols_per_step / (ms_per_step * 1e-3)
     eager = {"value": value, "ms_per_step": ms_per_step, "gpu_launches": int(launches)}
@@ -445,6 +465,8 @@ def main_gpu(args):
                 launches = gstep.last_launches * args.steps
                 clocks = clocks_g
                 graph_info = {"used": True, "kernels_per_replay": gstep.last_launches, "graph_launches_per_step": 1}
+                if args.dump_outputs:
+                    dump = snapshot()
             if world == 1:
                 for p in params:
                     p.grad = None
@@ -647,8 +669,29 @@ def main_gpu(args):
         "cpu_baseline": cpu,
     }
     print(json.dumps(line))
+    if dump is not None:
+        write_outputs(args.dump_outputs, dump)
     if world > 1:
         dist.destroy_process_group()
+
+
+DUMP_ARRAY_BYTES = 16 << 20      # per sampled array (H, agg); with the weight gradients the dump stays under 64 MB
+
+
+def sample_rows(x: torch.Tensor) -> np.ndarray:
+    """All rows of `x` as float32, or a fixed, seeded, sorted sample of them when they exceed DUMP_ARRAY_BYTES."""
+    x = x.detach().float()
+    cap = max(1, DUMP_ARRAY_BYTES // (4 * max(1, x.shape[1])))
+    if x.shape[0] > cap:
+        idx = np.sort(np.random.default_rng(0).choice(x.shape[0], size=cap, replace=False))
+        x = x[torch.from_numpy(idx).to(x.device)]
+    return x.cpu().numpy()
+
+
+def write_outputs(out_dir: str, arrays: dict):
+    os.makedirs(out_dir, exist_ok=True)
+    for k, v in arrays.items():
+        np.save(os.path.join(out_dir, f"{k}.npy"), np.ascontiguousarray(v, dtype=np.float32))
 
 
 def main():
@@ -666,7 +709,14 @@ def main():
     ap.add_argument("--no-dataset", action="store_true", help="(kept for old command lines; no effect)")
     ap.add_argument("--no-pack", action="store_true", help="keep the sampler's molecule order (no tile packing)")
     ap.add_argument("--no-graph", action="store_true", help="do not run the resident step as a CUDA graph")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last timed step computed (H, agg, loss, grad.<param>) "
+                         "as DIR/<name>.npy in float32")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be >= 1 and --warmup >= 0")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs applies to --impl b200")
     if args.impl == "reference":
         main_reference(args)
     else:

@@ -362,12 +362,93 @@ def mpnn_head_case() -> dict:
     return d
 
 
+# (kind, depth, bias, undirected, activation): the reference's own modules on the synthetic generator's molecules
+LIVE_CASES = [("bond", 3, False, False, "relu"), ("bond", 4, True, True, "elu"), ("atom", 3, True, False, "leakyrelu"),
+              ("atom", 2, False, False, "tanh"), ("bond", 1, False, False, "relu")]
+
+
+def live_case_name(kind: str, depth: int, bias: bool, undirected: bool, act: str) -> str:
+    return f"fixture_live_{kind}_d{depth}_{act}" + ("_bias" if bias else "") + ("_undirected" if undirected else "")
+
+
+def live_case_weights(shapes: dict, seed: int = 7) -> dict:
+    """Weights of a live case, by name (the module's state-dict keys, sorted): uniform in +-1/sqrt(fan_in), seeded, so that
+    the fixture needs no stored weights."""
+    rng = np.random.default_rng(seed)
+    out = {}
+    for k in sorted(shapes):
+        fan_in = shapes[k.replace(".bias", ".weight")][-1]
+        out[k] = rng.uniform(-1.0, 1.0, size=shapes[k]).astype(np.float32) / np.float32(np.sqrt(fan_in))
+    return out
+
+
+def live_sample(n: int, k: int, seed: int) -> np.ndarray:
+    """Sorted indices of a fixed sample of k out of n (all n when n <= k)."""
+    return np.arange(n) if n <= k else np.sort(np.random.default_rng(seed).choice(n, size=k, replace=False))
+
+
+def live_case(kind: str, depth: int, bias: bool, undirected: bool, act: str) -> dict:
+    """40 molecules of chemprop_b200.data.make_molecules(40, seed=11, shuffle_edges=True), collated by the reference's
+    BatchMolGraph (SHA-256 of each array); its {Bond,Atom}MessagePassing(d_h=96) holding live_case_weights(): H = mp(bmg),
+    its mean aggregation, and the weight gradients of loss = sum(mean_agg(H)^2) -- a fixed sample of the entries of each
+    (no entry for a weight without a gradient)."""
+    import hashlib
+
+    import_reference()
+    from chemprop.data import BatchMolGraph
+    from chemprop.data.molgraph import MolGraph
+    from chemprop.nn import AtomMessagePassing, BondMessagePassing, MeanAggregation
+
+    from chemprop_b200.data.synthetic import make_molecules
+
+    bmg = BatchMolGraph([MolGraph(*m) for m in make_molecules(40, seed=11, shuffle_edges=True)])
+    mp = (BondMessagePassing if kind == "bond" else AtomMessagePassing)(d_h=96, depth=depth, bias=bias,
+                                                                          undirected=undirected, activation=act)
+    W = live_case_weights({k: tuple(v.shape) for k, v in mp.state_dict().items()})
+    mp.load_state_dict({k: torch.from_numpy(v) for k, v in W.items()})
+    d = {"sha256." + k: hashlib.sha256(np.ascontiguousarray(getattr(bmg, k).numpy()).tobytes()).hexdigest()
+         for k in ("V", "E", "edge_index", "rev_edge_index", "batch")}
+    d["keys"] = " ".join(sorted(W))
+    H = mp(bmg)
+    a = MeanAggregation()(H, bmg.batch)
+    a.square().sum().backward()
+    d["rows.H_v"] = live_sample(H.shape[0], 24, 1)
+    d["H_v"] = H.detach().numpy()[d["rows.H_v"]]
+    d["agg_mean"] = a.detach().numpy()[live_sample(a.shape[0], 16, 2)]
+    for k, p in mp.named_parameters():
+        if p.grad is not None:
+            d["idx.grad." + k] = live_sample(p.grad.numel(), 512, 3)
+            d["grad." + k] = p.grad.numpy().reshape(-1)[d["idx.grad." + k]]
+    return d
+
+
+def seeded_sampler_case() -> dict:
+    """The reference's SeededSampler(203, seed=99): the sample order of two consecutive epochs."""
+    import_reference()
+    from chemprop.data.samplers import SeededSampler
+
+    s = SeededSampler(203, 99)
+    return {"order": np.stack([np.fromiter(iter(s), dtype=np.int64) for _ in range(2)]), "n": 203, "seed": 99}
+
+
 def main():
     """`python -m oracle.make_golden [name ...]`: all cases, or only the named ones (a case's seed is its position in
     CASES, so adding cases at the end never changes the committed ones)."""
     os.makedirs(GOLDEN_DIR, exist_ok=True)
     torch.set_num_threads(1)  # deterministic summation order
     only = set(sys.argv[1:])
+    for case in LIVE_CASES:
+        name = live_case_name(*case)
+        if name in only or not only:
+            np.savez_compressed(os.path.join(GOLDEN_DIR, f"{name}.npz"), **live_case(*case))
+            print(name)
+            only.discard(name)
+    if "fixture_seeded_sampler" in only or not only:
+        np.savez_compressed(os.path.join(GOLDEN_DIR, "fixture_seeded_sampler.npz"), **seeded_sampler_case())
+        print("fixture_seeded_sampler")
+        only.discard("fixture_seeded_sampler")
+    if not only and len(sys.argv) > 1:
+        return
     if "fixture_attentive" in only or not only:
         np.savez_compressed(os.path.join(GOLDEN_DIR, "fixture_attentive.npz"), **attentive_case())
         print("fixture_attentive")

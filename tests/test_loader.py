@@ -8,7 +8,7 @@ import torch
 
 from chemprop_b200.data import BatchMolGraph, PackedBatchLoader, PackedMolGraphDataset, make_molecules
 from chemprop_b200.data.loader import epoch_shard
-from oracle.ref_shim import reference_available
+from tests.util import load_golden
 
 N = 203
 
@@ -35,16 +35,11 @@ def test_seeded_order_is_the_references_seeded_sampler(data):
         got = np.concatenate([b.ids for b in loader])
         assert np.array_equal(got, idxs), epoch
     assert len(loader) == 7                                        # 203 = 6 * 32 + 11
-    if reference_available():
-        from oracle.ref_shim import import_reference
-
-        import_reference()
-        from chemprop.data.samplers import SeededSampler
-
-        ref = SeededSampler(N, 99)
-        ours = PackedBatchLoader(ds, batch_size=50, shuffle=True, seed=99, pack_tiles=False)
-        for _ in range(2):
-            assert np.array_equal(np.fromiter(iter(ref), dtype=np.int64), np.concatenate([b.ids for b in ours]))
+    ref = load_golden("fixture_seeded_sampler")                    # the reference's SeededSampler(203, 99), two epochs
+    assert int(ref["n"]) == N and int(ref["seed"]) == 99
+    ours = PackedBatchLoader(ds, batch_size=50, shuffle=True, seed=99, pack_tiles=False)
+    for epoch in range(2):
+        assert np.array_equal(ref["order"][epoch], np.concatenate([b.ids for b in ours])), epoch
 
 
 @pytest.mark.parametrize("prefetch,compact", [(2, False), (3, True)])

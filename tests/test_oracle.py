@@ -1,12 +1,11 @@
-"""CPU tier: pins oracle/restatement.py against the reference -- (1) every committed golden vector
-(produced by the unmodified reference, oracle/make_golden.py), (2) the live reference when the
-reference tree is reachable (it is not on the GPU box)."""
+"""CPU tier: pins oracle/restatement.py against the reference through the committed golden vectors and fixtures
+(produced by the unmodified reference, oracle/make_golden.py)."""
 import numpy as np
 import pytest
 import torch
 
 from oracle import layout_np, restatement as R
-from oracle.ref_shim import reference_available
+from oracle.make_golden import LIVE_CASES, live_case_name, live_case_weights, live_sample
 from tests.util import golden_names, load_golden, mab_oracle_forward, oracle_forward
 
 TOL = dict(rtol=1e-5, atol=1e-6)  # same torch ops on the same machine: differences are summation-order only
@@ -136,40 +135,37 @@ def test_layout_restatement_properties():
     assert Lb["max_tile_rows"] > 128 and Lb["n_tiles"] == 3
 
 
-@pytest.mark.skipif(not reference_available(), reason="reference tree not reachable (GPU box)")
-@pytest.mark.parametrize("kind,depth,bias,undirected,act", [
-    ("bond", 3, False, False, "relu"), ("bond", 4, True, True, "elu"), ("atom", 3, True, False, "leakyrelu"),
-    ("atom", 2, False, False, "tanh"), ("bond", 1, False, False, "relu"),
-])
+@pytest.mark.parametrize("kind,depth,bias,undirected,act", LIVE_CASES)
 def test_restatement_matches_live_reference(kind, depth, bias, undirected, act):
-    from oracle.ref_shim import import_reference
-
-    import_reference()
-    from chemprop.data import BatchMolGraph
-    from chemprop.data.molgraph import MolGraph
-    from chemprop.nn import AtomMessagePassing, BondMessagePassing, MeanAggregation
+    """The reference's own modules and collate on the synthetic generator's molecules (oracle/make_golden.py live_case):
+    the restated collate is bit-identical, and the restatement's hidden states, mean aggregation and weight gradients
+    match the reference's on the same weights."""
+    import hashlib
 
     from chemprop_b200.data.synthetic import make_molecules
+    from chemprop_b200.nn import AtomMessagePassing, BondMessagePassing
 
+    g = load_golden(live_case_name(kind, depth, bias, undirected, act))
     torch.set_num_threads(1)
-    torch.manual_seed(7)
     mgs = make_molecules(40, seed=11, shuffle_edges=True)
-    bmg = BatchMolGraph([MolGraph(*m) for m in mgs])
+    arrays = dict(zip(("V", "E", "edge_index", "rev_edge_index", "batch"), R.collate(mgs)))
+    for k, v in arrays.items():
+        assert hashlib.sha256(np.ascontiguousarray(v).tobytes()).hexdigest() == str(g["sha256." + k]), k
     cls = BondMessagePassing if kind == "bond" else AtomMessagePassing
-    mp = cls(d_h=96, depth=depth, bias=bias, undirected=undirected, activation=act)
-    H_ref = mp(bmg)
-    P = {k: v.detach().clone().requires_grad_(True) for k, v in mp.state_dict().items()}
-    H = R.message_passing_forward(kind, bmg.V, bmg.E, bmg.edge_index, bmg.rev_edge_index, P["W_i.weight"],
-                                  P.get("W_i.bias"), P["W_h.weight"], P.get("W_h.bias"), P["W_o.weight"],
-                                  P.get("W_o.bias"), depth, act, undirected)
-    torch.testing.assert_close(H, H_ref, **TOL)
-    a_ref = MeanAggregation()(H_ref, bmg.batch)
-    torch.testing.assert_close(R.aggregate(H, bmg.batch, "mean"), a_ref, **TOL)
-    a_ref.square().sum().backward()
-    R.aggregate(H, bmg.batch, "mean").square().sum().backward()
-    for k, p in mp.named_parameters():
-        torch.testing.assert_close(P[k].grad, p.grad, rtol=1e-4, atol=1e-6)
-    # and the reference's collate against the restated one
-    Vn, En, ein, revn, bn = R.collate(mgs)
-    assert np.array_equal(Vn, bmg.V.numpy()) and np.array_equal(ein, bmg.edge_index.numpy())
-    assert np.array_equal(revn, bmg.rev_edge_index.numpy()) and np.array_equal(bn, bmg.batch.numpy())
+    shapes = {k: tuple(v.shape) for k, v in cls(d_h=96, depth=depth, bias=bias, undirected=undirected,
+                                                  activation=act).state_dict().items()}
+    assert " ".join(sorted(shapes)) == str(g["keys"])                  # the engine module's state dict is the reference's
+    P = {k: torch.from_numpy(v).requires_grad_(True) for k, v in live_case_weights(shapes).items()}
+    V, E, ei, rev, batch = (torch.from_numpy(arrays[k]) for k in ("V", "E", "edge_index", "rev_edge_index", "batch"))
+    H = R.message_passing_forward(kind, V, E, ei, rev, P["W_i.weight"], P.get("W_i.bias"), P["W_h.weight"],
+                                  P.get("W_h.bias"), P["W_o.weight"], P.get("W_o.bias"), depth, act, undirected)
+    np.testing.assert_allclose(H.detach().numpy()[g["rows.H_v"]], g["H_v"], **TOL)
+    a = R.aggregate(H, batch, "mean")
+    np.testing.assert_allclose(a.detach().numpy()[live_sample(a.shape[0], 16, 2)], g["agg_mean"], **TOL)
+    a.square().sum().backward()
+    for k, p in P.items():
+        if "grad." + k not in g:
+            assert p.grad is None, k
+            continue
+        got = p.grad.numpy().reshape(-1)[g["idx.grad." + k]]
+        np.testing.assert_allclose(got, g["grad." + k], rtol=1e-4, atol=1e-6, err_msg=k)

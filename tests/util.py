@@ -117,7 +117,12 @@ class RecordingDropout(torch.nn.Dropout):
 
 def dropout_mask_for_mask(kind: str, undirected: bool, act: str, device: str, n_mols: int = 12, d_h: int = 32):
     """Training-mode dropout on the composed tier vs the oracle fed with the very masks the run drew (edge-level masks
-    mapped from the engine's dst-sorted row order back to the caller's edge order through `perm`)."""
+    mapped from the engine's dst-sorted row order back to the caller's edge order through `perm`).
+
+    An f32 pre-activation within rounding of an activation's kink (ReLU / PReLU at 0) can land on the other side of it
+    than its f64 counterpart, and one such element shifts whole gradient rows by its upstream gradient.  So the oracle
+    takes the engine's side of the kink at exactly those elements (its pre-activations, recorded in the same order,
+    mapped like the masks) -- and every one of them must agree with the oracle's pre-activation to the forward bound."""
     from chemprop_b200.data import BatchMolGraph, make_molecules
     from chemprop_b200.engine import get_layout
     from chemprop_b200.nn import AtomMessagePassing, BondMessagePassing, MeanAggregation
@@ -134,6 +139,8 @@ def dropout_mask_for_mask(kind: str, undirected: bool, act: str, device: str, n_
     assert mp.uses_composed_tier()
     V_d = torch.randn(bmg.V.shape[0], d_vd)
     P = {k: v.detach().double().requires_grad_(True) for k, v in mp.state_dict().items()}
+    pre = []                                      # the engine's activation inputs: H_0, every depth step, the read-out
+    mp.tau.register_forward_pre_hook(lambda mod, args: pre.append(args[0].detach().double().cpu()))
     mp = mp.to(device)
     bmg.to(device)
     H = mp(bmg, V_d.to(device))
@@ -148,15 +155,37 @@ def dropout_mask_for_mask(kind: str, undirected: bool, act: str, device: str, n_
         mm[perm] = m
         ref_masks.append(mm.double())
     ref_masks += [m.double() for m in masks[depth - 1:]]
+    assert len(pre) == depth + 1
+    for i in range(depth):                        # H_0 and the depth steps are edge-level, in the internal row order
+        z = torch.empty_like(pre[i])
+        z[perm] = pre[i]
+        pre[i] = z
+    base_tau = R.activation(act, P.get("tau.weight"))
+    kinks = []                                    # per activation call: elements where the oracle follows the engine's side
+
+    def tau(x):
+        z = pre[len(kinks)]
+        other_side = (x.detach() > 0) != (z > 0)
+        kinks.append((int(other_side.sum()), float((x.detach() - z)[other_side].abs().max()) if other_side.any() else 0.0))
+        return base_tau(x + torch.where(other_side, z - x.detach(), torch.zeros_like(z)))   # value shift only: d/dx = 1
+
     H_ref = R.message_passing_forward(kind, ref.V.double(), ref.E.double(), ref.edge_index, ref.rev_edge_index,
                                       P["W_i.weight"], P["W_i.bias"], P["W_h.weight"], P["W_h.bias"], P["W_o.weight"],
-                                      P["W_o.bias"], depth, act, undirected, V_d.double(), P["W_d.weight"], P["W_d.bias"],
-                                      prelu_weight=P.get("tau.weight"), dropout_masks=ref_masks)
+                                      P["W_o.bias"], depth, tau, undirected, V_d.double(), P["W_d.weight"], P["W_d.bias"],
+                                      dropout_masks=ref_masks)
     R.aggregate(H_ref, ref.batch, "mean").square().sum().backward()
+    assert len(kinks) == depth + 1 and max(d for _, d in kinks) <= 1e-5, kinks      # sides differ only within rounding
     assert (H.detach().double().cpu() - H_ref.detach()).abs().max().item() <= 1e-5
+    bad = {}
     for k, p in mp.named_parameters():
         g = P[k].grad
-        assert p.grad is not None and (p.grad.double().cpu() - g).abs().max().item() <= 1e-4 * max(1.0, g.abs().max().item()), k
+        assert p.grad is not None, k
+        d = (p.grad.double().cpu() - g).abs()
+        tol = 1e-4 * max(1.0, g.abs().max().item())
+        if d.max().item() > tol:       # every offending parameter: max error, bound, how many entries and which rows
+            bad[k] = (d.max().item(), tol, int((d > tol).sum()), sorted({int(i) for i in (d > tol).nonzero()[:, 0][:8]}))
+    assert not bad, (bad, kinks)
+    return kinks
 
 
 def mab_oracle_forward(g: dict, dtype=torch.float32, requires_grad: bool = False):
