@@ -85,6 +85,10 @@ SIGNATURES = {
     "dmpnn_bn_train_fwd": (C.c_int, [_vp, _i64, _i64, _i64, _vp, _vp, _f32, _f32, _vp, _vp, _vp, _i64, _vp, _i64, _vp, _vp, _vp]),
     "dmpnn_bn_bwd": (C.c_int, [_vp, _i64, _vp, _i64, _i64, _i64, _vp, _vp, _vp, _i64, _vp, _vp, _vp]),
     "dmpnn_mse_loss": (C.c_int, [_vp, _i64, _vp, _i64, _vp, _vp, _i64, _i64, _vp, _vp, _i64, _vp]),
+    "dmpnn_bce_loss": (C.c_int, [_vp, _i64, _vp, _i64, _vp, _vp, _i64, _i64, _vp, _vp, _i64, _vp]),
+    "dmpnn_ce_loss": (C.c_int, [_vp, _i64, _vp, _i64, _vp, _vp, _i64, _i64, _i64, _vp, _vp, _i64, _vp]),
+    "dmpnn_class_probs": (C.c_int, [_vp, _i64, _i64, _i64, _i64, _vp, _i64, _vp]),
+    "dmpnn_class_probs_bwd": (C.c_int, [_vp, _i64, _vp, _i64, _i64, _i64, _i64, _vp, _i64, _vp]),
 }
 
 

@@ -583,6 +583,47 @@ def mse_loss(P: Tensor, Y: Tensor, w, tw, loss: Tensor, dP: Tensor):
     _lib.check(rc, "dmpnn_mse_loss")
 
 
+def bce_loss(P: Tensor, Y: Tensor, w, tw, loss: Tensor, dP: Tensor):
+    """BCE with logits, P / Y / dP: B x T (dmpnn_bce_loss)."""
+    _require_cuda(P, Y, w, tw, loss, dP)
+    lib = _lib.load()
+    B, T = P.shape
+    rc = lib.dmpnn_bce_loss(P.data_ptr(), P.stride(0) if B else T, Y.data_ptr(), Y.stride(0) if B else T, _ptr(w), _ptr(tw), B, T,
+                            loss.data_ptr(), dP.data_ptr(), dP.stride(0) if B else T, _stream())
+    _lib.check(rc, "dmpnn_bce_loss")
+
+
+def ce_loss(P: Tensor, Y: Tensor, w, tw, loss: Tensor, dP: Tensor, C: int):
+    """Cross entropy over groups of C logits, P / dP: B x (T C), Y: B x T class ids (dmpnn_ce_loss)."""
+    _require_cuda(P, Y, w, tw, loss, dP)
+    lib = _lib.load()
+    B, T = Y.shape
+    TC = T * C
+    rc = lib.dmpnn_ce_loss(P.data_ptr(), P.stride(0) if B else TC, Y.data_ptr(), Y.stride(0) if B else T, _ptr(w), _ptr(tw), B, T,
+                           C, loss.data_ptr(), dP.data_ptr(), dP.stride(0) if B else TC, _stream())
+    _lib.check(rc, "dmpnn_ce_loss")
+
+
+def class_probs(P: Tensor, C: int, Q: Tensor):
+    """Q = sigmoid(P) (C == 1) or the softmax of each group of C columns, P / Q: B x (T C) (dmpnn_class_probs)."""
+    _require_cuda(P, Q)
+    lib = _lib.load()
+    B, TC = P.shape
+    rc = lib.dmpnn_class_probs(P.data_ptr(), P.stride(0) if B else TC, B, TC // C, C, Q.data_ptr(), Q.stride(0) if B else TC,
+                               _stream())
+    _lib.check(rc, "dmpnn_class_probs")
+
+
+def class_probs_bwd(Q: Tensor, dQ: Tensor, C: int, dP: Tensor):
+    """dP from the saved probabilities Q and the upstream dQ (dmpnn_class_probs_bwd)."""
+    _require_cuda(Q, dQ, dP)
+    lib = _lib.load()
+    B, TC = Q.shape
+    rc = lib.dmpnn_class_probs_bwd(Q.data_ptr(), Q.stride(0) if B else TC, dQ.data_ptr(), dQ.stride(0) if B else TC, B, TC // C, C,
+                                   dP.data_ptr(), dP.stride(0) if B else TC, _stream())
+    _lib.check(rc, "dmpnn_class_probs_bwd")
+
+
 def column_sum(Y: Tensor, R: int, N: int, out: Tensor, *, accumulate: bool = False):
     lib = _lib.load()
     n = C.c_size_t(0)

@@ -30,6 +30,9 @@ def register_with_chemprop() -> dict:
         ours.NormAggregation: ref_nn.NormAggregation,
         ours.AttentiveAggregation: ref_nn.AttentiveAggregation,
         ours.Aggregation: ref_nn.Aggregation,
+        # chemprop/cli/predict.py:509, 546 branch on isinstance(model.predictor, MulticlassClassificationFFN)
+        ours.EngineBinaryClassificationFFN: ref_nn.BinaryClassificationFFN,
+        ours.EngineMulticlassClassificationFFN: ref_nn.MulticlassClassificationFFN,
     }
     try:
         from chemprop.nn.ffn import ConstrainerFFN as ref_constrainer

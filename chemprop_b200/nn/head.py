@@ -1,12 +1,14 @@
 """Molecule-level head of the training step on the engine's kernels (SURVEY.md section 8f-2): what chemprop's `MPNN` does
 after the encoder -- `H = agg(H_v, batch)`, `H = bn(H)`, `preds = predictor(H)`, `loss = criterion(preds, targets, mask, w)`
 (chemprop/models/model.py:126-161, nn/ffn.py:38-61, nn/predictors.py:101-170, nn/metrics.py:78-123, 139-141) -- for the
-regression case: Mean / Sum / Norm aggregation, optional BatchNorm1d, the MLP of `RegressionFFN`, masked + weighted MSE.
+regression and classification cases: Mean / Sum / Norm aggregation, optional BatchNorm1d, the MLP of `RegressionFFN` /
+`BinaryClassificationFFN` / `MulticlassClassificationFFN`, masked + weighted MSE / BCE / cross entropy.
 
 Every arithmetic step is a libdmpnn launch (aggregation: dmpnn_segment_sum; batch norm: dmpnn_bn_train_fwd / dmpnn_bn_bwd;
 the MLP's GEMMs: dmpnn_linear_fwd / dmpnn_linear_wgrad with the activation in the epilogue; the criterion and its gradient:
-dmpnn_mse_loss), none synchronises with the host, so the encoder + head + backward (+ a capturable optimizer) replay as ONE CUDA
-graph (`chemprop_b200.graph.CudaGraphStep`).
+dmpnn_mse_loss / dmpnn_bce_loss / dmpnn_ce_loss; the classifiers' probabilities: dmpnn_class_probs), none synchronises with
+the host, so the encoder + head + backward (+ a capturable optimizer) replay as ONE CUDA graph
+(`chemprop_b200.graph.CudaGraphStep`).
 
 Module tree and state-dict keys are the reference's: `bn.{weight,bias,running_mean,running_var,num_batches_tracked}`,
 `predictor.ffn.<i>.<j>.{weight,bias}`, `predictor.criterion.task_weights` -- a reference `MPNN` state dict loads with
@@ -77,6 +79,79 @@ class MSELossFunction(torch.autograd.Function):
         return (dP * g).to(ctx.pdtype), None, None, None
 
 
+class BCELossFunction(torch.autograd.Function):
+    """chemprop's BCELoss on logits: sum(w_b * tw_t * mask * bce(z, y)) / sum(mask), mask = isfinite(targets); loss and
+    dLoss/dLogits in one launch (dmpnn_bce_loss)."""
+
+    @staticmethod
+    def forward(ctx, preds, targets, weights, task_weights):
+        K._require_cuda(preds, targets)
+        P, Y = preds.float().contiguous(), targets.float().contiguous()
+        w = None if weights is None else weights.float().reshape(-1).contiguous()
+        tw = None if task_weights is None else task_weights.float().reshape(-1).contiguous()
+        loss = torch.empty(1, device=P.device)
+        dP = torch.empty_like(P)
+        K.bce_loss(P, Y, w, tw, loss, dP)
+        ctx.save_for_backward(dP)
+        ctx.pdtype = preds.dtype
+        return loss.reshape(())
+
+    @staticmethod
+    def backward(ctx, g):
+        (dP,) = ctx.saved_tensors
+        return (dP * g).to(ctx.pdtype), None, None, None
+
+
+class CrossEntropyLossFunction(torch.autograd.Function):
+    """chemprop's CrossEntropyLoss on `b x t x C` logits and `b x t` class ids: sum(w_b * tw_t * mask * ce) / sum(mask);
+    loss and dLoss/dLogits in one launch (dmpnn_ce_loss).  An out-of-range class id gives a NaN loss (no host sync)."""
+
+    @staticmethod
+    def forward(ctx, preds, targets, weights, task_weights):
+        K._require_cuda(preds, targets)
+        if preds.dim() != 3 or tuple(preds.shape[:2]) != tuple(targets.shape):
+            raise ValueError(f"expected preds b x t x C and targets b x t, got {tuple(preds.shape)} and {tuple(targets.shape)}")
+        C = preds.shape[2]
+        P, Y = preds.float().reshape(preds.shape[0], -1).contiguous(), targets.float().contiguous()
+        w = None if weights is None else weights.float().reshape(-1).contiguous()
+        tw = None if task_weights is None else task_weights.float().reshape(-1).contiguous()
+        loss = torch.empty(1, device=P.device)
+        dP = torch.empty_like(P)
+        K.ce_loss(P, Y, w, tw, loss, dP, C)
+        ctx.save_for_backward(dP)
+        ctx.meta = (preds.dtype, preds.shape)
+        return loss.reshape(())
+
+    @staticmethod
+    def backward(ctx, g):
+        (dP,) = ctx.saved_tensors
+        dtype, shape = ctx.meta
+        return (dP.reshape(shape) * g).to(dtype), None, None, None
+
+
+class ClassProbsFunction(torch.autograd.Function):
+    """Eval output of the classification heads on `b x (t C)` logits: sigmoid (C == 1) or the softmax of each group of C
+    columns (dmpnn_class_probs); mirror from the saved probabilities (dmpnn_class_probs_bwd)."""
+
+    @staticmethod
+    def forward(ctx, logits, C):
+        K._require_cuda(logits)
+        P = logits.float().contiguous()
+        Q = torch.empty_like(P)
+        K.class_probs(P, C, Q)
+        ctx.save_for_backward(Q)
+        ctx.meta = (logits.dtype, C)
+        return Q
+
+    @staticmethod
+    def backward(ctx, dQ):
+        (Q,) = ctx.saved_tensors
+        dtype, C = ctx.meta
+        dP = torch.empty_like(Q)
+        K.class_probs_bwd(Q, dQ.float().contiguous(), C, dP)
+        return dP.to(dtype), None
+
+
 class LinearActFunction(torch.autograd.Function):
     """Y = act(X . W^T + b) with the activation in the GEMM epilogue (dmpnn_linear_fwd); mirror: dZ = dY * act'(Y)
     (dmpnn_act_bwd), dW / db (dmpnn_linear_wgrad), dX = dZ . W (dmpnn_linear_fwd)."""
@@ -124,6 +199,9 @@ class EngineLinear(nn.Linear):
 
 
 class _Criterion(nn.Module):
+    """chemprop's `ChempropMetric` call signature and `task_weights` buffer (1 x t); masked, weighted MSE."""
+    _function = MSELossFunction
+
     def __init__(self, task_weights):
         super().__init__()
         self.register_buffer("task_weights", torch.as_tensor(task_weights, dtype=torch.float).view(1, -1))
@@ -132,19 +210,29 @@ class _Criterion(nn.Module):
         if lt_mask is not None or gt_mask is not None:
             raise NotImplementedError("bounded MSE is not part of the engine's head; use the reference criterion")
         t = targets if mask is None else torch.where(mask, targets, torch.full_like(targets, float("nan")))
-        return MSELossFunction.apply(preds, t, weights, self.task_weights)
+        return self._function.apply(preds, t, weights, self.task_weights)
 
 
-class EngineRegressionFFN(nn.Module):
-    """`RegressionFFN` (chemprop/nn/predictors.py:156-164) with the reference's module tree; GEMMs on the engine."""
+class _BCECriterion(_Criterion):
+    """chemprop's `BCELoss` (nn/metrics.py:292-295): binary cross entropy on logits, soft labels accepted."""
+    _function = BCELossFunction
+
+
+class _CrossEntropyCriterion(_Criterion):
+    """chemprop's `CrossEntropyLoss` (nn/metrics.py:298-303): preds `b x t x C` logits, targets `b x t` class ids."""
+    _function = CrossEntropyLossFunction
+
+
+class _EngineFFN(nn.Module):
+    """The MLP of chemprop's `_FFNPredictorBase` (chemprop/nn/predictors.py:101-157) with the reference's module tree
+    (`ffn.<i>.<j>`, `criterion.task_weights`); GEMMs on the engine."""
     n_targets = 1
+    _criterion = _Criterion
 
-    def __init__(self, n_tasks: int = 1, input_dim: int = DEFAULT_HIDDEN_DIM, hidden_dim: int | Sequence[int] = 300,
-                 n_layers: int = 1, dropout: float = 0.0, activation="relu", task_weights=None):
+    def __init__(self, output_dim: int, n_tasks: int, input_dim: int, hidden_dim: int | Sequence[int], n_layers: int,
+                 dropout: float, activation, task_weights):
         super().__init__()
-        self.hparams = dict(n_tasks=n_tasks, input_dim=input_dim, hidden_dim=hidden_dim, n_layers=n_layers, dropout=dropout,
-                            activation=activation, cls=self.__class__)
-        ffn = build_mlp(input_dim, n_tasks, hidden_dim, n_layers, dropout, activation)
+        ffn = build_mlp(input_dim, output_dim, hidden_dim, n_layers, dropout, activation)
         for block in ffn:                         # same tree, engine-backed Linear layers
             for i, m in enumerate(block):
                 if isinstance(m, nn.Linear):
@@ -152,7 +240,7 @@ class EngineRegressionFFN(nn.Module):
                     e.load_state_dict(m.state_dict())
                     block[i] = e
         self.ffn = ffn
-        self.criterion = _Criterion(torch.ones(n_tasks) if task_weights is None else task_weights)
+        self.criterion = self._criterion(torch.ones(n_tasks) if task_weights is None else task_weights)
         self.output_transform = nn.Identity()
 
     @property
@@ -167,7 +255,7 @@ class EngineRegressionFFN(nn.Module):
     def n_tasks(self) -> int:
         return self.output_dim
 
-    def forward(self, Z: Tensor) -> Tensor:
+    def _mlp(self, Z: Tensor) -> Tensor:
         """`self.ffn(Z)` (nn/ffn.py:38-61: Linear, then [act, dropout, Linear] per further layer) with every activation the
         engine fuses folded into the epilogue of the GEMM before it."""
         blocks = [list(b) for b in self.ffn]
@@ -183,9 +271,66 @@ class EngineRegressionFFN(nn.Module):
             else:
                 X = tau(lin(X))
             X = drop(X)                                      # identity when p = 0 or in eval mode
-        return self.output_transform(X)
+        return X
+
+
+class EngineRegressionFFN(_EngineFFN):
+    """`RegressionFFN` (chemprop/nn/predictors.py:156-164) with the reference's module tree; GEMMs on the engine."""
+
+    def __init__(self, n_tasks: int = 1, input_dim: int = DEFAULT_HIDDEN_DIM, hidden_dim: int | Sequence[int] = 300,
+                 n_layers: int = 1, dropout: float = 0.0, activation="relu", task_weights=None):
+        super().__init__(n_tasks, n_tasks, input_dim, hidden_dim, n_layers, dropout, activation, task_weights)
+        self.hparams = dict(n_tasks=n_tasks, input_dim=input_dim, hidden_dim=hidden_dim, n_layers=n_layers, dropout=dropout,
+                            activation=activation, cls=self.__class__)
+
+    def forward(self, Z: Tensor) -> Tensor:
+        return self.output_transform(self._mlp(Z))
 
     train_step = forward
+
+
+class EngineBinaryClassificationFFN(_EngineFFN):
+    """`BinaryClassificationFFN` (chemprop/nn/predictors.py:235-247): `train_step` gives the `b x t` logits the BCE criterion
+    takes, `forward` their sigmoid (dmpnn_class_probs).  `threshold` is kept in `hparams` only, as in the reference, where
+    the BCE criterion ignores it."""
+    _criterion = _BCECriterion
+
+    def __init__(self, n_tasks: int = 1, input_dim: int = DEFAULT_HIDDEN_DIM, hidden_dim: int | Sequence[int] = 300,
+                 n_layers: int = 1, dropout: float = 0.0, activation="relu", task_weights=None, threshold: float | None = None):
+        super().__init__(n_tasks, n_tasks, input_dim, hidden_dim, n_layers, dropout, activation, task_weights)
+        self.hparams = dict(n_tasks=n_tasks, input_dim=input_dim, hidden_dim=hidden_dim, n_layers=n_layers, dropout=dropout,
+                            activation=activation, task_weights=task_weights, threshold=threshold, cls=self.__class__)
+
+    def forward(self, Z: Tensor) -> Tensor:
+        return ClassProbsFunction.apply(self._mlp(Z), 1)
+
+    def train_step(self, Z: Tensor) -> Tensor:
+        return self._mlp(Z)
+
+
+class EngineMulticlassClassificationFFN(_EngineFFN):
+    """`MulticlassClassificationFFN` (chemprop/nn/predictors.py:271-314): `n_tasks * n_classes` outputs; `train_step` gives
+    the `b x t x C` logits the cross-entropy criterion takes, `forward` the softmax over the classes (dmpnn_class_probs)."""
+    _criterion = _CrossEntropyCriterion
+
+    def __init__(self, n_classes: int, n_tasks: int = 1, input_dim: int = DEFAULT_HIDDEN_DIM,
+                 hidden_dim: int | Sequence[int] = 300, n_layers: int = 1, dropout: float = 0.0, activation="relu",
+                 task_weights=None, threshold: float | None = None):
+        super().__init__(n_tasks * n_classes, n_tasks, input_dim, hidden_dim, n_layers, dropout, activation, task_weights)
+        self.n_classes = n_classes
+        self.hparams = dict(n_classes=n_classes, n_tasks=n_tasks, input_dim=input_dim, hidden_dim=hidden_dim,
+                            n_layers=n_layers, dropout=dropout, activation=activation, task_weights=task_weights,
+                            threshold=threshold, cls=self.__class__)
+
+    @property
+    def n_tasks(self) -> int:
+        return self.output_dim // (self.n_targets * self.n_classes)
+
+    def forward(self, Z: Tensor) -> Tensor:
+        return ClassProbsFunction.apply(self._mlp(Z), self.n_classes).reshape(Z.shape[0], -1, self.n_classes)
+
+    def train_step(self, Z: Tensor) -> Tensor:
+        return self._mlp(Z).reshape(Z.shape[0], -1, self.n_classes)
 
 
 class EngineBatchNorm1d(nn.BatchNorm1d):

@@ -432,6 +432,19 @@ int dmpnn_wgrad_x3(const float* dY, int64_t lddy, const float* X, int64_t ldx, i
  *   dmpnn_bn_bwd        dX (and dgamma, dbeta when non-null) from dY, Xhat, invstd.
  *   dmpnn_mse_loss      chemprop's MSE criterion (nn/metrics.py:78-123, 139-141): loss[0] = sum_{b,t} w[b] tw[t] m (P - Y)^2
  *                       / sum m with m = isfinite(Y) (NaN target = masked, model.py:140-141); dP (nullable) = dloss/dP.
+ *   dmpnn_bce_loss      chemprop's BCELoss on logits (nn/metrics.py:292-295): P, Y are B x T; per element
+ *                       L = max(z, 0) - z y + log1p(exp(-|z|)) (soft labels in [0, 1] accepted);
+ *                       loss[0] = sum w[b] tw[t] m L / sum m; dP (nullable) = w tw m (sigmoid(z) - y) / sum m.
+ *   dmpnn_ce_loss       chemprop's CrossEntropyLoss (nn/metrics.py:298-303): P is B x (T C), column t C + c = logit of class
+ *                       c of task t (predictors.py: reshape(b, -1, C)); Y is B x T class ids; L = logsumexp(z) - z_y;
+ *                       dP (nullable) = w tw m (softmax(z) - onehot(y)) / sum m.  A finite target that is not an integer
+ *                       in [0, C) makes loss[0] (and that item's dP) NaN: the stand-in for torch's error, which would
+ *                       need a host sync.
+ *                       For both: m = isfinite(Y); loss[0] = 0 and dP = 0 when sum m = 0.  One cluster of 8 blocks
+ *                       (partials combined in rank order over distributed shared memory): bit-reproducible.
+ *   dmpnn_class_probs   eval output of the classification heads (predictors.py:241-244, 310-311): Q = sigmoid(P) when
+ *                       C == 1, otherwise softmax over each group of C columns; P, Q are B x (T C).
+ *   dmpnn_class_probs_bwd  dP = dQ q (1 - q) (C == 1) or q (dQ - <dQ, q>) per group, from the saved Q.
  * All reductions run in a fixed order (deterministic); no host synchronisation.
  * ------------------------------------------------------------------------------------- */
 int dmpnn_bn_train_fwd(const float* X, int64_t ldx, int64_t B, int64_t d, const float* gamma, const float* beta,
@@ -442,6 +455,14 @@ int dmpnn_bn_bwd(const float* dY, int64_t lddy, const float* Xhat, int64_t ldh, 
                  void* stream);
 int dmpnn_mse_loss(const float* P, int64_t ldp, const float* Y, int64_t ldy, const float* weights,
                    const float* task_weights, int64_t B, int64_t T, float* loss, float* dP, int64_t lddp, void* stream);
+int dmpnn_bce_loss(const float* P, int64_t ldp, const float* Y, int64_t ldy, const float* weights,
+                   const float* task_weights, int64_t B, int64_t T, float* loss, float* dP, int64_t lddp, void* stream);
+int dmpnn_ce_loss(const float* P, int64_t ldp, const float* Y, int64_t ldy, const float* weights,
+                  const float* task_weights, int64_t B, int64_t T, int64_t C, float* loss, float* dP, int64_t lddp,
+                  void* stream);
+int dmpnn_class_probs(const float* P, int64_t ldp, int64_t B, int64_t T, int64_t C, float* Q, int64_t ldq, void* stream);
+int dmpnn_class_probs_bwd(const float* Q, int64_t ldq, const float* dQ, int64_t lddq, int64_t B, int64_t T, int64_t C,
+                          float* dP, int64_t lddp, void* stream);
 
 #ifdef __cplusplus
 }
